@@ -169,10 +169,11 @@ __device__ __forceinline__ float4 ld_dsmem_f4(uint32_t remote) {
   return v;
 }
 
-// a kernel launch with a cluster dimension along x (and the programmatic-dependent-launch attribute)
+// a kernel launch in thread-block clusters of shape `cluster` (and the programmatic-dependent-launch attribute); returns
+// what cudaLaunchKernelEx returned
 template <typename... KArgs, typename... Args>
-inline void launch_k_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, unsigned cluster_x,
-                             Args&&... args) {
+inline cudaError_t launch_k_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, dim3 cluster,
+                                    Args&&... args) {
   if (trace_host_armed()) trace_host_launch(reinterpret_cast<const void*>(kernel), grid, block, stream);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
@@ -181,14 +182,14 @@ inline void launch_k_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = cluster_x;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
+  attr[0].val.clusterDim.x = cluster.x;
+  attr[0].val.clusterDim.y = cluster.y;
+  attr[0].val.clusterDim.z = cluster.z;
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
   cfg.attrs = attr;
   cfg.numAttrs = 2;
-  cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 __device__ __forceinline__ uint32_t smem_addr_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ float ld_dsmem_f32(uint32_t remote) {

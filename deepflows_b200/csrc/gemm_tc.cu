@@ -34,6 +34,7 @@
 #include <cuda.h>
 
 #include <algorithm>
+#include <type_traits>
 
 namespace dfb {
 namespace tc {
@@ -566,7 +567,9 @@ struct SmemLayout {
   // [4 warps][4 values][BN columns]
   static constexpr uint32_t kEpiOffset = kBarOffset + kOverRead + kNumBars * 8 + 16;
   static constexpr uint32_t kEpiBytes = 1024 + 64 * BN;
-  static constexpr uint32_t kOutOffset = (kEpiOffset + 16 + kEpiBytes + 48 + 15) & ~15u;   // (+48: the persistent kernel's three extra barriers)
+  // the persistent kernel's accumulator barriers: full[2], empty[2] (32 bytes of the 48 reserved)
+  static constexpr uint32_t kAccBarOffset = (kEpiOffset + 16 + kEpiBytes + 15) & ~15u;
+  static constexpr uint32_t kOutOffset = kAccBarOffset + 48;
   static constexpr uint32_t kTotal = kOutOffset + kOutBytes + 1024;  // +1024 for manual alignment
   // split-K partial tile staged in the (idle) pipeline stages: 128 rows, padded pitch against bank conflicts
   static constexpr uint32_t kRedPitch = BN + 4;
@@ -575,22 +578,25 @@ struct SmemLayout {
   static constexpr bool kFits = kTotal <= 227u * 1024u;
   static_assert(XMUL > 1 || kFits, "more shared memory than a CTA can have");
 };
+// the layout of tc_kernel<P, X3> (OUT = false) and tc_persistent_kernel<P, X3> (OUT = true)
+template <class P, bool OUT, bool X3>
+using TcLayout = SmemLayout<P::BN, P::AROWS, P::KR, P::kBSub, P::BKR, OUT, X3 ? 2 : 1>;
 
 // X3 = true: fp32-accurate contraction on the tensor pipe ("3xTF32", the package's default fp32 mode). TMA delivers fp32
-// operands; the four epilogue warps, idle during the main loop, split every stage in shared memory into a TF32-exact high
-// part (written back in place: hi = rna_tf32(v)) and a low part (lo = rna_tf32(v - hi), the second half of the stage), and
-// the MMA warp issues hi*hi + lo*hi + hi*lo into the same fp32 accumulator. What is dropped is lo*lo and the rounding of
-// lo: <= 2^-21 per product relative to |a||b| - the size of fp32's own accumulation error (measured against the fp64
-// contraction in tests/test_gpu_l1.py), and independent of how the hardware rounds fp32 operands to TF32.
-// Replaces the FFMA kernels of gemm_simt.cu as what an unchanged script runs (reference kernel being replaced:
-// ndarray_backend_cuda.cu:443-466).
+// operands; warps that are idle during the main loop split every stage in shared memory into a TF32-exact high part
+// (written back in place: hi = rna_tf32(v)) and a low part (lo = rna_tf32(v - hi), the second half of the stage), and the
+// MMA warp issues hi*hi into the accumulator and lo*hi + hi*lo into a second, small-term accumulator (see tc_kernel) that
+// the epilogue adds. What is dropped is lo*lo and the rounding of lo: <= 2^-21 per product relative to |a||b| - the size
+// of fp32's own accumulation error (measured against the fp64 contraction in tests/test_gpu_l1.py), and independent of how
+// the hardware rounds fp32 operands to TF32. Replaces the FFMA kernels of gemm_simt.cu as what an unchanged script runs
+// (reference kernel being replaced: ndarray_backend_cuda.cu:443-466).
 __device__ __forceinline__ float rna_tf32(float v) {
   uint32_t r;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));
   return __uint_as_float(r);
 }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive_cta(uint64_t* bar) {
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
@@ -599,7 +605,7 @@ __global__ void __launch_bounds__(kThreads) tc_kernel(const __grid_constant__ CU
                                                       const __grid_constant__ CUtensorMap map_b,
                                                       const typename P::Params prm) {
   constexpr int BN = P::BN;
-  using L = SmemLayout<BN, P::AROWS, P::KR, P::kBSub, P::BKR, false, X3 ? 2 : 1>;
+  using L = TcLayout<P, false, X3>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + L::kBarOffset + L::kOverRead);
@@ -710,8 +716,8 @@ __global__ void __launch_bounds__(kThreads) tc_kernel(const __grid_constant__ CU
 #pragma unroll
           for (int t = 0; t < P::kSubTiles; ++t) {
             const uint32_t a_sub = a_base + P::a_sub_offset(prm, t), b_sub = b_base + P::b_sub_offset(prm, t, L::kBTile);
-            const uint32_t d_tmem = tmem_base + (uint32_t)(t * P::kAccStride);  // kAccStride == 0: one shared accumulator
-            const uint32_t first = (kb > kb_begin || (P::kAccStride == 0 && t > 0) || j > 0) ? 1u : 0u;
+            const uint32_t d_tmem = tmem_base;
+            const uint32_t first = (kb > kb_begin || t > 0 || j > 0) ? 1u : 0u;
 #pragma unroll
             for (int term = 0; term < (X3 ? 3 : 1); ++term) {   // hi*hi, lo*hi, hi*lo (the low parts: + kStageBytes)
               const uint32_t a_op = a_sub + (term == 1 ? L::kStageBytes : 0u), b_op = b_sub + (term == 2 ? L::kStageBytes : 0u);
@@ -755,7 +761,7 @@ __global__ void __launch_bounds__(kThreads) tc_kernel(const __grid_constant__ CU
         }
         fence_proxy_async_smem();   // generic-proxy writes -> visible to the tensor core's (async proxy) operand reads
         __syncwarp();
-        if (elect_one()) mbar_arrive_cta(split_bar + stage);
+        if (elect_one()) mbar_arrive(split_bar + stage);
         __syncwarp();
         if (++stage == kStages) { stage = 0; phase ^= 1; }
       }
@@ -936,9 +942,6 @@ __global__ void __launch_bounds__(kThreads) tc_kernel(const __grid_constant__ CU
 // tile boundaries, the MMA warp alternates between two TMEM accumulators, and the epilogue warps drain accumulator i
 // (TMEM -> dedicated staging tile -> coalesced stores, statistics in registers across ALL tiles of the CTA: one partial
 // per CTA) while the MMAs of tile i + 1 run. Row-major problems without split-K only.
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 // X3 (fp32-accurate form, see tc_kernel): four more warps (6-9) split every stage into its TF32 high / low parts - the
 // epilogue warps are busy with the previous tile here - and each of the two accumulators has a second one for the small terms.
 template <class P, bool X3 = false>
@@ -946,8 +949,10 @@ __global__ void __launch_bounds__(X3 ? kThreads + 128 : kThreads) tc_persistent_
                                                                                        const __grid_constant__ CUtensorMap map_b,
                                                                                        const typename P::Params prm, const int n_tiles) {
   constexpr int BN = P::BN;
-  static_assert(P::kRowMajor && P::kAccTiles == 1 && P::kAccStride == 0, "persistent kernel: row-major, one accumulator tile");
-  using L = SmemLayout<BN, P::AROWS, P::KR, P::kBSub, P::BKR, true, X3 ? 2 : 1>;
+  static_assert(P::kRowMajor && P::kAccTiles == 1 && P::kMmaN == BN && P::kTmemCols == BN,
+                "persistent kernel: row-major, one accumulator tile of BN columns (the two accumulators are kAccW apart)");
+  static_assert(!P::kRuntimeLbo, "persistent kernel: compile-time operand descriptors");
+  using L = TcLayout<P, true, X3>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + L::kBarOffset + L::kOverRead);
@@ -958,7 +963,7 @@ __global__ void __launch_bounds__(X3 ? kThreads + 128 : kThreads) tc_persistent_
   (void)split_bar;
   float** row_tab = reinterpret_cast<float**>(smem + ((L::kEpiOffset + 15) & ~15u));
   float* wstat = reinterpret_cast<float*>(row_tab + BLOCK_M);
-  uint64_t* tmem_full_bar = reinterpret_cast<uint64_t*>(smem + L::kOutOffset - 48);   // [2] full, [2] empty
+  uint64_t* tmem_full_bar = reinterpret_cast<uint64_t*>(smem + L::kAccBarOffset);   // [2] full, [2] empty
   uint64_t* tmem_empty_bar = tmem_full_bar + 2;
   constexpr int kAccW = X3 ? 2 * BN : BN;               // columns of one accumulator (X3: + the small-term accumulator)
   constexpr int kAccCols = 2 * kAccW < 32 ? 32 : 2 * kAccW;   // two accumulators (BN is a power of two >= 32)
@@ -1073,7 +1078,7 @@ __global__ void __launch_bounds__(X3 ? kThreads + 128 : kThreads) tc_persistent_
           }
           fence_proxy_async_smem();
           __syncwarp();
-          if (elect_one()) mbar_arrive_cta(split_bar + stage);
+          if (elect_one()) mbar_arrive(split_bar + stage);
           __syncwarp();
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
@@ -1484,89 +1489,64 @@ static bool make_map(CUtensorMap* map, const float* base, int rank, const uint64
 // fp32-accurate mode of the current call (set by the tc_* entry points): launch() then picks tc_kernel<P, true>
 static thread_local bool g_x3 = false;
 template <class P>
-static constexpr bool x3_fits() { return SmemLayout<P::BN, P::AROWS, P::KR, P::kBSub, P::BKR, false, 2>::kFits; }
+static constexpr bool x3_fits() { return TcLayout<P, false, true>::kFits; }
 
-template <class P, bool X3>
-static dfb_status launch_variant(const char* name, const CUtensorMap& ma, const CUtensorMap& mb, const typename P::Params& prm,
-                                 dim3 grid, int splits) {
-  using L = SmemLayout<P::BN, P::AROWS, P::KR, P::kBSub, P::BKR, false, X3 ? 2 : 1>;
+// Launches a tcgen05 kernel on the compute stream: sets its dynamic shared-memory size on the first call, launches
+// (split_k_cluster: the `splits` CTAs that share a tile form one cluster along z; grid.z already counts them), checks and
+// counts the launch.
+template <auto Kernel, typename... Args>
+static dfb_status launch_tc(const char* name, dim3 grid, unsigned threads, uint32_t smem, bool split_k_cluster, int splits,
+                            const Args&... args) {
   static bool configured = false;
   if (!configured) {
-    DFB_CUDA(cudaFuncSetAttribute(tc_kernel<P, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::kTotal));
+    DFB_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
-  if (P::kClusterSplit) {
-    // grid.z already counts the splits; the S CTAs that share a tile form one cluster along z
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(kThreads, 1, 1);
-    cfg.dynamicSmemBytes = L::kTotal;
-    cfg.stream = compute_stream();
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = (unsigned)splits;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-    cfg.attrs = attr;
-    cfg.numAttrs = 2;
-    if (trace_host_armed()) trace_host_launch(reinterpret_cast<const void*>(tc_kernel<P, X3>), grid, dim3(kThreads, 1, 1), cfg.stream);
-    cudaError_t e = cudaLaunchKernelEx(&cfg, tc_kernel<P, X3>, ma, mb, prm);
+  if (split_k_cluster) {
+    const cudaError_t e = launch_k_cluster(Kernel, grid, threads, smem, compute_stream(), dim3(1, 1, (unsigned)splits), args...);
     if (e != cudaSuccess) {
       cudaGetLastError();
       DFB_FAIL(DFB_ERR_RUNTIME, "%s cluster launch (splits %d) failed: %s", name, splits, cudaGetErrorString(e));
     }
   } else {
-    launch_k(tc_kernel<P, X3>, grid, kThreads, L::kTotal, compute_stream(), ma, mb, prm);
+    launch_k(Kernel, grid, threads, smem, compute_stream(), args...);
   }
   DFB_LAUNCH_CHECK(name);
   g_tc_launches.fetch_add(1, std::memory_order_relaxed);
   return DFB_OK;
 }
+// one tile per CTA; grid.z already counts the splits
 template <class P>
 static dfb_status launch(const char* name, const CUtensorMap& ma, const CUtensorMap& mb, const typename P::Params& prm,
                          dim3 grid, int splits = 1) {
   if (g_x3) {
     if constexpr (x3_fits<P>()) {
-      return launch_variant<P, true>(name, ma, mb, prm, grid, splits);
+      return launch_tc<tc_kernel<P, true>>(name, grid, kThreads, TcLayout<P, false, true>::kTotal, P::kClusterSplit, splits, ma, mb, prm);
     } else {
       DFB_FAIL(DFB_ERR_RUNTIME, "%s: this tile variant has no fp32-accurate form (host selection error)", name);
     }
   }
-  return launch_variant<P, false>(name, ma, mb, prm, grid, splits);
+  return launch_tc<tc_kernel<P, false>>(name, grid, kThreads, TcLayout<P, false, false>::kTotal, P::kClusterSplit, splits, ma, mb, prm);
 }
 
-template <class P, bool X3>
-static dfb_status launch_persistent_variant(const char* name, const CUtensorMap& ma, const CUtensorMap& mb, const typename P::Params& prm,
-                                            int n_tiles, unsigned ctas) {
-  using L = SmemLayout<P::BN, P::AROWS, P::KR, P::kBSub, P::BKR, true, X3 ? 2 : 1>;
-  static bool configured = false;
-  if (!configured) {
-    DFB_CUDA(cudaFuncSetAttribute(tc_persistent_kernel<P, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::kTotal));
-    configured = true;
-  }
-  launch_k(tc_persistent_kernel<P, X3>, dim3(ctas, 1, 1), X3 ? kThreads + 128 : kThreads, L::kTotal, compute_stream(), ma, mb, prm, n_tiles);
-  DFB_LAUNCH_CHECK(name);
-  g_tc_launches.fetch_add(1, std::memory_order_relaxed);
-  return DFB_OK;
-}
 // fp32-accurate form only where two CTAs still share an SM (the grid is sized for that): the kernels without row halo
 template <class P>
 static constexpr bool x3_persistent_ok() {
-  return P::kSubTiles == 1 && SmemLayout<P::BN, P::AROWS, P::KR, P::kBSub, P::BKR, true, 2>::kTotal <= 113u * 1024u;
+  return P::kSubTiles == 1 && TcLayout<P, true, true>::kTotal <= 113u * 1024u;
 }
 template <class P>
 static dfb_status launch_persistent(const char* name, const CUtensorMap& ma, const CUtensorMap& mb, const typename P::Params& prm,
                                     int n_tiles, unsigned ctas) {
   if (g_x3) {
     if constexpr (x3_persistent_ok<P>()) {
-      return launch_persistent_variant<P, true>(name, ma, mb, prm, n_tiles, ctas);
+      return launch_tc<tc_persistent_kernel<P, true>>(name, dim3(ctas, 1, 1), kThreads + 128, TcLayout<P, true, true>::kTotal, false, 1, ma, mb,
+                                                      prm, n_tiles);
     } else {
       DFB_FAIL(DFB_ERR_RUNTIME, "%s: no fp32-accurate persistent form of this variant (host selection error)", name);
     }
   }
-  return launch_persistent_variant<P, false>(name, ma, mb, prm, n_tiles, ctas);
+  return launch_tc<tc_persistent_kernel<P, false>>(name, dim3(ctas, 1, 1), kThreads, TcLayout<P, true, false>::kTotal, false, 1, ma, mb, prm,
+                                                   n_tiles);
 }
 // DFB_CONV_PERSISTENT=0 switches the persistent variant off (every tile its own CTA again)
 static bool persistent_enabled() {
@@ -1590,20 +1570,11 @@ static bool wide_enabled() {
 template <class P, int EF>
 static dfb_status launch_wide(const char* name, const CUtensorMap& ma, const CUtensorMap& mb, const typename P::Params& prm, int n_tiles,
                               int col_tiles) {
-  using W = WideLayout<P>;
-  static bool configured = false;
-  if (!configured) {
-    DFB_CUDA(cudaFuncSetAttribute(tc_wide_kernel<P, EF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)W::kTotal));
-    configured = true;
-  }
   // whole waves: every CTA walks the same number of tiles (+-1)
   const int sms = sm_count();
   const int waves = (n_tiles + sms - 1) / sms;
   const unsigned ctas = (unsigned)((n_tiles + waves - 1) / waves);
-  launch_k(tc_wide_kernel<P, EF>, dim3(ctas, 1, 1), kThreads, W::kTotal, compute_stream(), ma, mb, prm, n_tiles, col_tiles);
-  DFB_LAUNCH_CHECK(name);
-  g_tc_launches.fetch_add(1, std::memory_order_relaxed);
-  return DFB_OK;
+  return launch_tc<tc_wide_kernel<P, EF>>(name, dim3(ctas, 1, 1), kThreads, WideLayout<P>::kTotal, false, 1, ma, mb, prm, n_tiles, col_tiles);
 }
 
 // Split-K factor (cluster size along z, a power of two <= 8): enough CTAs to occupy the machine, at least
@@ -1630,7 +1601,7 @@ template <int A_MAJ, int B_MAJ, int BN_>
 struct GemmProblem {
   static constexpr int BN = BN_, A_MAJOR = A_MAJ, B_MAJOR = B_MAJ;
   static constexpr bool kClusterSplit = true;
-  static constexpr int AROWS = BLOCK_M, KR = BLOCK_K, BKR = BLOCK_K, kSubTiles = 1, kBSub = 1, kAccStride = 0, kAccTiles = 1, kTmemCols = BN_;
+  static constexpr int AROWS = BLOCK_M, KR = BLOCK_K, BKR = BLOCK_K, kSubTiles = 1, kBSub = 1, kAccTiles = 1, kTmemCols = BN_;
   __device__ static uint32_t a_sub_offset(const GemmParams&, int) { return 0; }
   __device__ static uint32_t b_sub_offset(const GemmParams&, int, uint32_t) { return 0; }
   static constexpr int kMmaN = BN_;
@@ -1789,7 +1760,7 @@ struct ConvProblem {
   static constexpr int BN = BN_, A_MAJOR = MAJOR_K, B_MAJOR = (WMODE == W_KRSC_DGRAD ? MAJOR_MN : MAJOR_K);
   static constexpr bool kClusterSplit = true;
   static constexpr int AROWS = ROWS ? 192 : BLOCK_M, KR = BLOCK_K, BKR = BLOCK_K, kSubTiles = ROWS ? 3 : 1, kBSub = kSubTiles;
-  static constexpr int kAccStride = 0, kAccTiles = 1, kTmemCols = BN_;
+  static constexpr int kAccTiles = 1, kTmemCols = BN_;
   using LayoutT = SmemLayout<BN_, AROWS, KR, kBSub, BKR>;
   __device__ static uint32_t b_sub_offset(const ConvParams&, int t, uint32_t b_tile) { return t * b_tile; }
   static constexpr int kMmaN = BN_;
@@ -1951,7 +1922,7 @@ struct WgradProblem {
   // row-halo: the three taps are the three 32-wide chunks of ONE N = 3 * BN operand (chunk stride = ow_t rows), so
   // a k-step is one MMA, not three (with N = 32 the MMA issue latency, not the math, is what a k-step costs)
   static constexpr int kSubTiles = 1, kBSub = 1;
-  static constexpr int kAccTiles = ROWS_ ? 3 : 1, kAccStride = 0, kMmaN = ROWS_ ? 3 * BN_ : BN_;
+  static constexpr int kAccTiles = ROWS_ ? 3 : 1, kMmaN = ROWS_ ? 3 * BN_ : BN_;
   static constexpr int kTmemCols = ROWS_ ? (BN_ * 3 <= 128 ? 128 : (BN_ * 3 <= 256 ? 256 : 512)) : BN_;
   static constexpr bool kRuntimeLbo = ROWS_;
   static_assert(!ROWS_ || BN_ == 32, "the row-halo wgrad addresses taps as operand chunks: one 32-wide chunk per tap");
@@ -2249,6 +2220,30 @@ static bool make_act_map(CUtensorMap* map, const float* base, int N, int H, int 
   return make_map(map, base, 5, d, s, b, major);
 }
 
+// The epilogue work of a convolution (EF_* flags) -> the EF template argument, for every kernel family. Only the
+// combinations the host asks for are instantiated: fprop + statistics, dgrad + addend / BatchNorm-backward sums (with or
+// without the ReLU mask) / both, with channels-last weights. conv_like refuses the others (fprop with an addend or
+// BatchNorm-backward sums, dgrad with statistics, any fused epilogue with packed weights); should one arrive anyway, the
+// flags a pass has no variant for are dropped: fprop keeps only EF_STATS, dgrad ignores EF_STATS, packed weights get
+// EF_NONE.
+template <int WMODE, class F>
+static dfb_status with_conv_epilogue(int ef, F&& launch_ef) {
+  using std::integral_constant;
+  if constexpr (WMODE == W_KRSC_FPROP) {
+    if (ef & EF_STATS) return launch_ef(integral_constant<int, EF_STATS>());
+  } else if constexpr (WMODE == W_KRSC_DGRAD) {
+    switch (ef & ~EF_STATS) {
+      case EF_BNBWD | EF_RELU | EF_ADDEND: return launch_ef(integral_constant<int, EF_BNBWD | EF_RELU | EF_ADDEND>());
+      case EF_BNBWD | EF_RELU: return launch_ef(integral_constant<int, EF_BNBWD | EF_RELU>());
+      case EF_BNBWD | EF_ADDEND: return launch_ef(integral_constant<int, EF_BNBWD | EF_ADDEND>());
+      case EF_BNBWD: return launch_ef(integral_constant<int, EF_BNBWD>());
+      case EF_ADDEND: return launch_ef(integral_constant<int, EF_ADDEND>());
+      default: break;
+    }
+  }
+  return launch_ef(integral_constant<int, EF_NONE>());
+}
+
 template <int BN, int WMODE, bool ROWS = false>
 static dfb_status run_conv(const char* name, const CUtensorMap& ma, const float* wt, int n_out, int taps, int cp, int K, int C,
                            ConvParams prm, bool* handled) {
@@ -2285,9 +2280,9 @@ static dfb_status run_conv(const char* name, const CUtensorMap& ma, const float*
     prm.epi.stat_part = part;
     prm.epi.stat_cnt = part + partials * 3 * n_out;
   }
-  // the epilogue work is a template parameter; only the combinations the host asks for exist: fprop + statistics,
-  // dgrad + addend / BatchNorm-backward sums / both (channels-last weights; conv_like refuses the rest)
   const bool add = prm.epi.addend != nullptr;
+  const int ef = (prm.epi.stat_kind == EPI_STATS ? EF_STATS : 0) | (add ? EF_ADDEND : 0) |
+                 (prm.epi.stat_kind == EPI_BNBWD ? EF_BNBWD | (prm.epi.relu ? EF_RELU : 0) : 0);
   dfb_status st = DFB_OK;
   bool launched = false;
   // Many more tiles than CTA slots, one column tile, no split: CTAs that live for the whole launch (tc_persistent_kernel),
@@ -2302,17 +2297,9 @@ static dfb_status run_conv(const char* name, const CUtensorMap& ma, const float*
         prm.epi.stat_cnt = part + (size_t)ctas * 3 * n_out;
       }
       grid = dim3(ctas, 1, 1);
-      if constexpr (WMODE == W_KRSC_FPROP) {
-        if (prm.epi.stat_kind == EPI_STATS) st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_STATS>>(name, ma, mb, prm, n_tiles, ctas);
-        else st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_NONE>>(name, ma, mb, prm, n_tiles, ctas);
-      } else {
-        if (prm.epi.stat_kind == EPI_BNBWD && prm.epi.relu && add) st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_BNBWD | EF_RELU | EF_ADDEND>>(name, ma, mb, prm, n_tiles, ctas);
-        else if (prm.epi.stat_kind == EPI_BNBWD && prm.epi.relu) st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_BNBWD | EF_RELU>>(name, ma, mb, prm, n_tiles, ctas);
-        else if (prm.epi.stat_kind == EPI_BNBWD && add) st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_BNBWD | EF_ADDEND>>(name, ma, mb, prm, n_tiles, ctas);
-        else if (prm.epi.stat_kind == EPI_BNBWD) st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_BNBWD>>(name, ma, mb, prm, n_tiles, ctas);
-        else if (add) st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_ADDEND>>(name, ma, mb, prm, n_tiles, ctas);
-        else st = launch_persistent<ConvProblem<BN, WMODE, ROWS, EF_NONE>>(name, ma, mb, prm, n_tiles, ctas);
-      }
+      st = with_conv_epilogue<WMODE>(ef, [&](auto e) {
+        return launch_persistent<ConvProblem<BN, WMODE, ROWS, decltype(e)::value>>(name, ma, mb, prm, n_tiles, ctas);
+      });
       launched = true;
     }
   }
@@ -2322,36 +2309,14 @@ static dfb_status run_conv(const char* name, const CUtensorMap& ma, const float*
     const int n_tiles = (int)(grid.x * grid.y), col_tiles = (int)grid.y;
     const bool slot_ok = prm.epi.stat_kind == EPI_NONE || prm.epi.stat_acc != nullptr;
     if (wide_enabled() && !g_x3 && classes == 1 && prm.splits == 1 && slot_ok && n_out <= 512 && (size_t)n_tiles >= (size_t)sm_count() * 2) {
-#define DFB_WIDE(EFV) st = launch_wide<ConvProblem<BN, WMODE, ROWS, (EFV)>, (EFV)>(name, ma, mb, prm, n_tiles, col_tiles)
-      if constexpr (WMODE == W_KRSC_FPROP) {
-        if (prm.epi.stat_kind == EPI_STATS) DFB_WIDE(EF_STATS);
-        else DFB_WIDE(EF_NONE);
-      } else if constexpr (WMODE == W_KRSC_DGRAD) {
-        if (prm.epi.stat_kind == EPI_BNBWD && prm.epi.relu && add) DFB_WIDE(EF_BNBWD | EF_RELU | EF_ADDEND);
-        else if (prm.epi.stat_kind == EPI_BNBWD && prm.epi.relu) DFB_WIDE(EF_BNBWD | EF_RELU);
-        else if (prm.epi.stat_kind == EPI_BNBWD && add) DFB_WIDE(EF_BNBWD | EF_ADDEND);
-        else if (prm.epi.stat_kind == EPI_BNBWD) DFB_WIDE(EF_BNBWD);
-        else if (add) DFB_WIDE(EF_ADDEND);
-        else DFB_WIDE(EF_NONE);
-      } else {
-        DFB_WIDE(EF_NONE);
-      }
-#undef DFB_WIDE
+      st = with_conv_epilogue<WMODE>(ef, [&](auto e) {
+        return launch_wide<ConvProblem<BN, WMODE, ROWS, decltype(e)::value>, decltype(e)::value>(name, ma, mb, prm, n_tiles, col_tiles);
+      });
       launched = true;
     }
   }
-  if constexpr (WMODE == W_KRSC_FPROP) {
-    if (!launched && prm.epi.stat_kind == EPI_STATS) { st = launch<ConvProblem<BN, WMODE, ROWS, EF_STATS>>(name, ma, mb, prm, grid, prm.splits); launched = true; }
-  }
-  if constexpr (WMODE == W_KRSC_DGRAD) {
-    if (launched) {
-    } else if (prm.epi.stat_kind == EPI_BNBWD && prm.epi.relu && add) { st = launch<ConvProblem<BN, WMODE, ROWS, EF_BNBWD | EF_RELU | EF_ADDEND>>(name, ma, mb, prm, grid, prm.splits); launched = true; }
-    else if (prm.epi.stat_kind == EPI_BNBWD && prm.epi.relu) { st = launch<ConvProblem<BN, WMODE, ROWS, EF_BNBWD | EF_RELU>>(name, ma, mb, prm, grid, prm.splits); launched = true; }
-    else if (prm.epi.stat_kind == EPI_BNBWD && add) { st = launch<ConvProblem<BN, WMODE, ROWS, EF_BNBWD | EF_ADDEND>>(name, ma, mb, prm, grid, prm.splits); launched = true; }
-    else if (prm.epi.stat_kind == EPI_BNBWD) { st = launch<ConvProblem<BN, WMODE, ROWS, EF_BNBWD>>(name, ma, mb, prm, grid, prm.splits); launched = true; }
-    else if (add) { st = launch<ConvProblem<BN, WMODE, ROWS, EF_ADDEND>>(name, ma, mb, prm, grid, prm.splits); launched = true; }
-  }
-  if (!launched) st = launch<ConvProblem<BN, WMODE, ROWS, EF_NONE>>(name, ma, mb, prm, grid, prm.splits);
+  if (!launched)
+    st = with_conv_epilogue<WMODE>(ef, [&](auto e) { return launch<ConvProblem<BN, WMODE, ROWS, decltype(e)::value>>(name, ma, mb, prm, grid, prm.splits); });
   if (st == DFB_OK && part) {
     launch_k(epi_finalize_kernel, (unsigned)(n_out / 4), 128, 0, compute_stream(), (const float*)prm.epi.stat_part, (const float*)prm.epi.stat_cnt,
              (int)(grid.x * grid.z), n_out, prm.epi.stat_kind == EPI_STATS ? 1 : 0, prm.epi.stat_out);

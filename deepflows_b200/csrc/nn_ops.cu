@@ -1414,7 +1414,7 @@ dfb_status dfb_bn_fwd_train(const float* x, const float* gamma, const float* bet
   if (const int gpb = sp.gpb) {
     const unsigned grid = (unsigned)(C / 4 / gpb) * sp.cluster;
     cudaStream_t s = compute_stream();
-#define DFB_BN_SMALL_FWD(G) launch_k_cluster(bn_small_fwd_kernel<G>, grid, kSmallT, 0, s, sp.cluster, x, gamma, beta, y, save_mean, \
+#define DFB_BN_SMALL_FWD(G) launch_k_cluster(bn_small_fwd_kernel<G>, grid, kSmallT, 0, s, dim3(sp.cluster, 1, 1), x, gamma, beta, y, save_mean, \
                                              save_invstd, running_mean, running_var, momentum, eps, (int)rows, C)
     if (gpb == 1) DFB_BN_SMALL_FWD(1);
     else if (gpb == 2) DFB_BN_SMALL_FWD(2);
@@ -1458,7 +1458,7 @@ dfb_status dfb_bn_bwd(const float* x, const float* dy, const float* gamma, const
   if (const int gpb = sp.gpb) {
     const unsigned grid = (unsigned)(C / 4 / gpb) * sp.cluster;
     cudaStream_t s = compute_stream();
-#define DFB_BN_SMALL_BWD(G) launch_k_cluster(bn_small_bwd_kernel<G>, grid, kSmallT, 0, s, sp.cluster, x, dy, gamma, save_mean, \
+#define DFB_BN_SMALL_BWD(G) launch_k_cluster(bn_small_bwd_kernel<G>, grid, kSmallT, 0, s, dim3(sp.cluster, 1, 1), x, dy, gamma, save_mean, \
                                              save_invstd, dx, dgamma, dbeta, (int)rows, C)
     if (gpb == 1) DFB_BN_SMALL_BWD(1);
     else if (gpb == 2) DFB_BN_SMALL_BWD(2);

@@ -7,7 +7,7 @@ out=deepflows_b200/lib/obj_timing
 mkdir -p $out
 flags="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 --expt-relaxed-constexpr -DDFB_TC_TIMING"
 pids=()
-for f in runtime ewise gemm_simt gemm_tc conv_direct gemm nn_ops data_ops optim comm; do
+for f in runtime ewise gemm_simt gemm_tc conv_direct gemm nn_ops data_ops optim comm peer; do
   if [ ! -f $out/$f.o ] || [ deepflows_b200/csrc/$f.cu -nt $out/$f.o ] || [ "$f" = gemm_tc ]; then
     nvcc $flags -c deepflows_b200/csrc/$f.cu -o $out/$f.o &
     pids+=($!)
