@@ -7,6 +7,8 @@ implemented as ONE graph node over the device's fused (L1) entry points.
     max_pool2d      reference: pad + im2col + row max, equality-mask backward [347-374, tensor.py:779-791]
                     ->  one forward kernel, one backward kernel with the same tie semantics
     avg_pool2d      reference raises AttributeError [377-404] (SURVEY Q4)  ->  implemented
+    conv_transpose2d  absent in the reference  ->  the convolution's dgrad / fprop / wgrad kernels with roles swapped
+    interpolate     absent in the reference  ->  nearest / bilinear upsampling kernels, forward and backward
     cross_entropy   reference: 10 tensor ops [104-115]  ->  fused softmax-CE forward / backward
     batch_norm      reference: 16 tensor ops inside BatchNorm2d.forward [modules/batchnorm.py:30-55]
     relu            reference: maximum(x, 0) [15-16]  ->  same forward kernel, one-kernel backward
@@ -254,6 +256,54 @@ def _lazy(dev):
     return (True,) if dev.has("STATS_LAZY") else ()
 
 
+def _conv_weight(kernel: Tensor, dev):
+    """(weight data, WLAYOUT_*) of a (K,C,R,R) convolution weight as the convolution kernels take it.
+    Weights live channels-last (K,R,R,C) on the B200 device - the layout the tensor-core kernels read
+    in place, for fprop and (as the transposed operand) for dgrad. A Parameter that arrives compact
+    (fresh from init / load_state_dict / a checkpoint) is re-laid out once, here; its logical shape,
+    `.numpy()` and every other consumer are unaffected (strides carry the layout)."""
+    wd = kernel.data
+    if wd.ndim == 4 and wd.is_channels_last():
+        return wd, WLAYOUT_KRSC
+    if (wd.ndim == 4 and dev.name == "cuda" and dev.has("WLAYOUT_KRSC")
+            and not isinstance(kernel, (UnaryOperator, BinaryOperator, FusedOperator))):  # a stored tensor, not an op result
+        kernel.data = wd = wd.channels_last()
+        return wd, WLAYOUT_KRSC
+    return wd.compact(), WLAYOUT_KCRS
+
+
+def _workspace(dev, geom):
+    n_floats = dev.conv2d_workspace_floats(*geom)
+    return (dev.Array(n_floats), n_floats) if n_floats else (None, 0)
+
+
+def _wgrad_beside_dgrad(dev, needs, weight: Tensor, wgrad, dgrad):
+    """Runs the weight gradient `wgrad()` (when needs[1]) and returns the input gradient `dgrad()` (when needs[0], else
+    None) of a convolution-like op. The two only share their inputs: when both are needed the weight gradient goes to the
+    side stream and the two kernels (neither fills 148 SMs on the small layers) run concurrently."""
+    both = needs[0] and needs[1] and dev.has("side_begin") and _SIDE_STREAM
+    # The weight gradient is read by nobody before the end of backward() (Tensor.backward joins the side stream there;
+    # DeepFlows.dist joins before it packs a bucket), so the compute stream only waits for the weight gradient of
+    # _SIDE_LAG layers ago: wgrad overlaps the next layers' dgrad / BatchNorm chain instead of sitting on it. Not when
+    # the weight already holds a gradient (shared weights, accumulation): the sum would read dw right away.
+    lazy_join = both and _SIDE_LAG > 0 and dev.has("side_join_lag") and weight.grad is None
+    if needs[1]:
+        if both:
+            dev.side_begin()
+        try:
+            wgrad()
+        finally:
+            if both:
+                dev.side_end()
+    dx = dgrad() if needs[0] else None
+    if both:
+        if lazy_join:
+            dev.side_join_lag(_SIDE_LAG)
+        else:
+            dev.side_join()
+    return dx
+
+
 class _conv2d(FusedOperator):
     def __init__(self, x: Tensor, kernel: Tensor, padding: int, stride: int, want_stats: bool = False):
         self.padding, self.stride = int(padding), int(stride)
@@ -261,20 +311,9 @@ class _conv2d(FusedOperator):
         super().__init__(x, kernel)
 
     def forward(self, x, kernel):
-        xd, wd = x.data, kernel.data
+        xd = x.data
         dev = xd.device
-        # Weights live channels-last (K,R,R,C) on the B200 device - the layout the tensor-core kernels read
-        # in place, for fprop and (as the transposed operand) for dgrad. A Parameter that arrives compact
-        # (fresh from init / load_state_dict / a checkpoint) is re-laid out once, here; its logical shape,
-        # `.numpy()` and every other consumer are unaffected (strides carry the layout).
-        if wd.ndim == 4 and wd.is_channels_last():
-            w_layout = WLAYOUT_KRSC
-        elif (wd.ndim == 4 and dev.name == "cuda" and dev.has("WLAYOUT_KRSC")
-              and not isinstance(kernel, (UnaryOperator, BinaryOperator, FusedOperator))):  # a stored tensor, not an op result
-            kernel.data = wd = wd.channels_last()
-            w_layout = WLAYOUT_KRSC
-        else:
-            wd, w_layout = wd.compact(), WLAYOUT_KCRS
+        wd, w_layout = _conv_weight(kernel, dev)
         n, c, h, w = xd.shape
         k, c2, r, r2 = wd.shape
         assert c == c2 and r == r2, "conv2d: kernel %s does not match input %s" % (wd.shape, xd.shape)
@@ -316,46 +355,31 @@ class _conv2d(FusedOperator):
             out = _nhwc_view(y, n, k, oh, ow, dev)
             out._aux = ("colstats", mean_var)
             return out
-        ws, ws_n = self._workspace(dev)
+        ws, ws_n = _workspace(dev, self._geom)
         dev.conv2d_fprop(xd._handle, layout, wd._handle, y, n, c, h, w, k, r, p, s, mode, ws, ws_n, *self._wl)
         return _nhwc_view(y, n, k, oh, ow, dev)
-
-    def _workspace(self, dev):
-        n_floats = dev.conv2d_workspace_floats(*self._geom)
-        return (dev.Array(n_floats), n_floats) if n_floats else (None, 0)
 
     def backward_all(self, grad, needs):
         n, c, h, w, k, r, p, s = self._geom
         dev = self._x.device
         gy = grad.channels_last()
-        ws, ws_n = self._workspace(dev)
-        dx = dw = None
-        # dgrad and wgrad only share their inputs: when both are needed the wgrad goes to the side stream
-        # and the two kernels (neither fills 148 SMs on the small layers) run concurrently
-        both = needs[0] and needs[1] and dev.has("side_begin") and _SIDE_STREAM
-        # The weight gradient is read by nobody before the end of backward() (Tensor.backward joins the side stream there;
-        # DeepFlows.dist joins before it packs a bucket), so the compute stream only waits for the weight gradient of
-        # _SIDE_LAG layers ago: wgrad overlaps the next layers' dgrad / BatchNorm chain instead of sitting on it. Not when
-        # the weight already holds a gradient (shared weights, accumulation): the sum would read dw right away.
-        lazy_join = both and _SIDE_LAG > 0 and dev.has("side_join_lag") and self.inputs[1].grad is None
+        ws, ws_n = _workspace(dev, self._geom)
+        dw = None
         if needs[1]:
             # the weight gradient is produced in the weight's own layout, so optimizer and all-reduce walk
             # the two buffers side by side
             dw = _nhwc_view(dev.Array(k * c * r * r), k, c, r, r, dev) if self._wl else BackendTensor.make((k, c, r, r), device=dev)
-            if both:
-                dev.side_begin()
-            try:
-                if self._col is not None:   # first layer: the column matrix of the forward pass is still there
-                    col, oh, ow, cols = self._col
-                    dev.conv2d_wgrad_cols(col, gy._handle, dw._handle, self._wl[0] if self._wl else WLAYOUT_KCRS, n, oh, ow, k, cols,
-                                          self._mode)
-                else:
-                    dev.conv2d_wgrad(self._x._handle, self._layout, gy._handle, dw._handle, n, c, h, w, k, r, p, s,
-                                     self._mode, ws, ws_n, *self._wl)
-            finally:
-                if both:
-                    dev.side_end()
-        if needs[0]:
+
+        def wgrad():
+            if self._col is not None:   # first layer: the column matrix of the forward pass is still there
+                col, oh, ow, cols = self._col
+                dev.conv2d_wgrad_cols(col, gy._handle, dw._handle, self._wl[0] if self._wl else WLAYOUT_KCRS, n, oh, ow, k, cols,
+                                      self._mode)
+            else:
+                dev.conv2d_wgrad(self._x._handle, self._layout, gy._handle, dw._handle, n, c, h, w, k, r, p, s,
+                                 self._mode, ws, ws_n, *self._wl)
+
+        def dgrad():
             buf = dev.Array(n * h * w * c)
             dmode = 0 if get_dgrad_mode() == "reference" else 1
             fuse = self._dgrad_fusion(dev, n, c, h, w) if (dmode == 1 and get_fusion() and dev.has("conv2d_dgrad_fused")) else None
@@ -376,12 +400,9 @@ class _conv2d(FusedOperator):
                 dev.conv2d_dgrad(gy._handle, self._w._handle, buf, n, c, h, w, k, r, p, s, self._mode, dmode, ws, ws_n,
                                  *self._wl)
                 dx = _nhwc_view(buf, n, c, h, w, dev)
-        if both:
-            if lazy_join:
-                dev.side_join_lag(_SIDE_LAG)
-            else:
-                dev.side_join()
-        return dx, dw
+            return dx
+
+        return _wgrad_beside_dgrad(dev, needs, self.inputs[1], wgrad, dgrad), dw
 
     def _dgrad_fusion(self, dev, n, c, h, w):
         """What the dgrad epilogue can take over for the input tensor x of this convolution:
@@ -435,6 +456,102 @@ def conv2d(x: Tensor, kernel: Tensor, padding: int = 0, stride: int = 1, want_st
     if not isinstance(x, Tensor):
         x = Tensor(x, device=kernel.device)
     return _conv2d(x, kernel, padding, stride, want_stats)
+
+
+def check_conv_transpose2d_args(padding: int, stride: int, output_padding: int):
+    """ValueError unless stride >= 1, padding >= 0 and 0 <= output_padding < stride - under that condition a convolution
+    with the same kernel size, stride and padding maps the transposed convolution's output size back to its input size."""
+    if stride < 1 or padding < 0:
+        raise ValueError("conv_transpose2d: stride must be >= 1 and padding >= 0 (got stride=%d, padding=%d)" % (stride, padding))
+    if not 0 <= output_padding < stride:
+        raise ValueError("conv_transpose2d: output_padding must satisfy 0 <= output_padding < stride (got %d, stride %d)"
+                         % (output_padding, stride))
+
+
+def conv_transpose2d_size(h_in: int, kernel_size: int, padding: int, stride: int, output_padding: int) -> int:
+    """Output height (or width) of a transposed convolution: (h_in - 1) * stride - 2 * padding + kernel_size + output_padding
+    (arguments checked by check_conv_transpose2d_args; ValueError for an empty output)."""
+    check_conv_transpose2d_args(padding, stride, output_padding)
+    h = (h_in - 1) * stride - 2 * padding + kernel_size + output_padding
+    if h < 1:
+        raise ValueError("conv_transpose2d: input size %d, kernel %d, padding %d, stride %d give an empty output"
+                         % (h_in, kernel_size, padding, stride))
+    return h
+
+
+class _conv_transpose2d(FusedOperator):
+    """The transposed convolution of x (N,in,H,W) with weight (in,out,k,k) is the input gradient of the convolution
+    conv2d(., weight, padding, stride) - K = in, C = out in the notation of the convolution entry points - so every pass
+    runs on that convolution's kernels:
+        forward        y  = conv2d_dgrad(x, w)              (always DGRAD_EXACT: the transposed convolution itself)
+        d/dx           dx = conv2d_fprop(dy, w)
+        d/dw           dw = conv2d_wgrad(x = dy, dy = x)    (in the weight's own layout, on the side stream)"""
+
+    def __init__(self, x: Tensor, kernel: Tensor, padding: int, stride: int, output_padding: int):
+        self.padding, self.stride, self.output_padding = int(padding), int(stride), int(output_padding)
+        super().__init__(x, kernel)
+
+    def forward(self, x, kernel):
+        xd = x.data.channels_last()
+        dev = xd.device
+        wd, w_layout = _conv_weight(kernel, dev)
+        n, k, hi, wi = xd.shape
+        k2, c, r, r2 = wd.shape
+        assert k == k2 and r == r2, "conv_transpose2d: weight %s does not match input %s" % (wd.shape, xd.shape)
+        p, s, op = self.padding, self.stride, self.output_padding
+        h, w = conv_transpose2d_size(hi, r, p, s, op), conv_transpose2d_size(wi, r, p, s, op)
+        self._geom = (n, c, h, w, k, r, p, s)
+        self._x, self._w, self._mode = xd, wd, precision_mode()
+        self._wl = (w_layout,) if w_layout else ()
+        ws, ws_n = _workspace(dev, self._geom)
+        y = dev.Array(n * h * w * c)
+        dev.conv2d_dgrad(xd._handle, wd._handle, y, n, c, h, w, k, r, p, s, self._mode, 1, ws, ws_n, *self._wl)
+        return _nhwc_view(y, n, c, h, w, dev)
+
+    def backward_all(self, grad, needs):
+        n, c, h, w, k, r, p, s = self._geom
+        dev = self._x.device
+        hi, wi = self._x.shape[2:]
+        gy = grad.channels_last()
+        ws, ws_n = _workspace(dev, self._geom)
+        dw = None
+        if needs[1]:
+            dw = _nhwc_view(dev.Array(k * c * r * r), k, c, r, r, dev) if self._wl else BackendTensor.make((k, c, r, r), device=dev)
+
+        def wgrad():
+            dev.conv2d_wgrad(gy._handle, LAYOUT_NHWC, self._x._handle, dw._handle, n, c, h, w, k, r, p, s, self._mode, ws, ws_n,
+                             *self._wl)
+
+        def dgrad():
+            buf = dev.Array(n * hi * wi * k)
+            dev.conv2d_fprop(gy._handle, LAYOUT_NHWC, self._w._handle, buf, n, c, h, w, k, r, p, s, self._mode, ws, ws_n, *self._wl)
+            return _nhwc_view(buf, n, k, hi, wi, dev)
+
+        return _wgrad_beside_dgrad(dev, needs, self.inputs[1], wgrad, dgrad), dw
+
+    def release(self):
+        self._x = self._w = None
+
+
+def conv_transpose2d(x: Tensor, weight: Tensor, padding: int = 0, stride: int = 1, output_padding: int = 0):
+    """2-d transposed convolution, x (N,in,H,W), weight (in,out,k,k) as in PyTorch -> (N,out,H_out,W_out) with
+    H_out = (H - 1) * stride - 2 * padding + k + output_padding, 0 <= output_padding < stride. Square kernel, no
+    dilation / groups. The positional order is this package's conv2d order - padding before stride - which a positional
+    call written for torch.nn.functional.conv_transpose2d (stride, padding, output_padding) would misread.
+
+    It is the input gradient of conv2d with the same weight, padding and stride, and runs on that convolution's kernels:
+      * forward on the tensor pipe (tcgen05) in TF32 and fp32 mode when in % 4 == 0, out % 4 == 0, stride 1 or 2, and for
+        stride 2 an even output size (k = 4 / p = 1, k = 2 / p = 0, k = 3 / p = 1 / output_padding = 1); odd stride-2 outputs
+        (k = 3, p = 1, output_padding = 0), channel counts that are not multiples of 4 and stride >= 3 run on the exact FFMA
+        kernels;
+      * backward with respect to x: conv2d_fprop(dy, weight), and with respect to the weight: conv2d_wgrad with x and dy
+        swapped - for an image-producing layer (out <= 4, out * k * k <= 80, in a multiple of 16 up to 64) both through the
+        exact direct kernels of conv_direct.cu that serve the first layer of a convolutional network.
+    The exact transposed convolution is computed whatever `set_dgrad_mode` says (that switch selects the reference's
+    last-writer-wins quirk for Conv2d's backward only)."""
+    if not isinstance(x, Tensor):
+        x = Tensor(x, device=weight.device)
+    return _conv_transpose2d(x, weight, padding, stride, output_padding)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -504,6 +621,79 @@ class _pool2d(FusedOperator):
 
     def release(self):
         self._x = self._y = None
+
+
+UPSAMPLE_NEAREST, UPSAMPLE_BILINEAR = 0, 1   # include/dfb200.h: DFB_UPSAMPLE_*
+_UPSAMPLE_MODES = {"nearest": UPSAMPLE_NEAREST, "bilinear": UPSAMPLE_BILINEAR}
+_UPSAMPLE_MAX_SCALE = 8
+
+
+class _upsample2d(FusedOperator):
+    """(N,C,H,W) -> (N,C,H*s,W*s) by an integer factor s, one channels-last kernel each way (dfb_upsample2d_fwd / _bwd)."""
+
+    def __init__(self, x: Tensor, scale: int, mode: int):
+        self.scale, self.mode = int(scale), int(mode)
+        super().__init__(x)
+
+    def forward(self, x):
+        xd = x.data.channels_last()
+        n, c, h, w = xd.shape
+        dev = xd.device
+        s = self.scale
+        y = dev.Array(n * h * s * w * s * c)
+        dev.upsample2d_fwd(xd._handle, y, n, h, w, c, s, self.mode)
+        self._shape, self._dev = (n, c, h, w), dev
+        return _nhwc_view(y, n, c, h * s, w * s, dev)
+
+    def backward_all(self, grad, needs):
+        n, c, h, w = self._shape
+        dev = self._dev
+        gy = grad.channels_last()
+        dx = dev.Array(n * h * w * c)
+        dev.upsample2d_bwd(gy._handle, dx, n, h, w, c, self.scale, self.mode)
+        return (_nhwc_view(dx, n, c, h, w, dev),)
+
+    def release(self):
+        self._dev = None
+
+
+def _integer_scale(v, what):
+    """An integer upsampling factor from a number or a pair of equal numbers, else NotImplementedError."""
+    if isinstance(v, (tuple, list)):
+        if len(v) != 2 or v[0] != v[1]:
+            raise NotImplementedError("interpolate: %s %r: only the same factor for height and width is supported" % (what, v))
+        v = v[0]
+    if isinstance(v, bool) or not isinstance(v, (int, float)) or v != int(v) or not 1 <= int(v) <= _UPSAMPLE_MAX_SCALE:
+        raise NotImplementedError("interpolate: %s %r: only integer factors from 1 to %d are supported"
+                                  % (what, v, _UPSAMPLE_MAX_SCALE))
+    return int(v)
+
+
+def interpolate(input: Tensor, size=None, scale_factor=None, mode: str = "nearest", align_corners=None):
+    """Upsampling of an (N,C,H,W) tensor by an integer factor s (1..8, the same for H and W), torch.nn.functional.interpolate's
+    arguments: `scale_factor` = s, or `size` = (H*s, W*s) (an int for both axes). Modes "nearest" (a copy of the source pixel
+    (oh // s, ow // s)) and "bilinear" with align_corners=False (PyTorch's half-pixel rule, edges clamped). Other modes,
+    align_corners=True and non-integer or per-axis factors raise NotImplementedError; malformed arguments ValueError."""
+    if mode not in _UPSAMPLE_MODES:
+        raise NotImplementedError("interpolate: mode %r is not supported (nearest, bilinear)" % (mode,))
+    if align_corners is not None and mode == "nearest":
+        raise ValueError("interpolate: align_corners can only be set with the interpolating mode 'bilinear'")
+    if align_corners:
+        raise NotImplementedError("interpolate: align_corners=True is not supported (align_corners=False / None is)")
+    if input.ndim != 4:
+        raise ValueError("interpolate: expected an (N,C,H,W) input, got shape %s" % (input.shape,))
+    if (size is None) == (scale_factor is None):
+        raise ValueError("interpolate: give exactly one of size and scale_factor")
+    h, w = input.shape[2:]
+    if scale_factor is not None:
+        s = _integer_scale(scale_factor, "scale_factor")
+    else:
+        oh, ow = (size, size) if isinstance(size, int) else tuple(size)
+        if oh % h or ow % w or oh // h != ow // w:
+            raise NotImplementedError("interpolate: size %r is not the same integer multiple of the input size (%d, %d)"
+                                      % (size, h, w))
+        s = _integer_scale(oh // h, "size / input size")
+    return _upsample2d(input, s, _UPSAMPLE_MODES[mode])
 
 
 class _pad_spatial(UnaryOperator):

@@ -66,3 +66,24 @@ class Conv2d(_ConvNd):
         # per-channel statistics of the output, which BatchNorm then does not have to compute (F.batch_norm)
         out = F.conv2d(x, self.weight, self.padding, self.stride, want_stats=self.bias is None and self.training)
         return out + self.bias if self.bias is not None else out
+
+
+class ConvTranspose2d(_ConvNd):
+    """Transposed convolution, weight (in_channels, out_channels, k, k) as in PyTorch's ConvTranspose2d, bias
+    (1, out_channels, 1, 1); output size (H - 1) * stride - 2 * padding + k + output_padding, 0 <= output_padding < stride.
+    The positional order is this package's Conv2d order - padding before stride, then output_padding - not PyTorch's
+    (stride, padding, output_padding): pass them by keyword when porting a model. Initialisation is Conv2d's; fan_in is
+    read from shape[1] = out_channels * k * k, as PyTorch does for this layer. See F.conv_transpose2d for the kernels."""
+
+    def __init__(self, in_channels: int, out_channels: int, kernel_size: int, padding: int = 0, stride: int = 1,
+                 output_padding: int = 0, bias: bool = True, device="cuda", dtype=None) -> None:
+        super().__init__()
+        F.check_conv_transpose2d_args(padding, stride, output_padding)
+        self.in_channels, self.out_channels, self.kernel_size = in_channels, out_channels, kernel_size
+        self.padding, self.stride, self.output_padding = padding, stride, output_padding
+        self._make_params((in_channels, out_channels, kernel_size, kernel_size), (1, out_channels, 1, 1), bias,
+                          device, dtype)
+
+    def forward(self, x):
+        out = F.conv_transpose2d(x, self.weight, self.padding, self.stride, self.output_padding)
+        return out + self.bias if self.bias is not None else out

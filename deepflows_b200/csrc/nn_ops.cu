@@ -1031,6 +1031,142 @@ avgpool_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, int N, 
 }
 
 // -------------------------------------------------------------------------------------------------
+// upsampling by an integer factor s on NHWC: x [N,H,W,C] -> y [N,H*s,W*s,C]. Both backward kernels gather (one thread per
+// input pixel sums, in a fixed order, every output gradient that read it): no atomics, so results do not depend on scheduling.
+// -------------------------------------------------------------------------------------------------
+template <int V>
+__global__ void __launch_bounds__(kT)
+upsample_nearest_fwd_kernel(const float* __restrict__ x, float* __restrict__ y, int N, int H, int W, int C, int s) {
+  pdl_sync();
+  const int G = C / V, OH = H * s, OW = W * s;
+  size_t total = (size_t)N * OH * OW * G;
+  size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    int g = (int)(i % G);
+    size_t t = i / G;
+    int ow = (int)(t % OW);
+    t /= OW;
+    int oh = (int)(t % OH);
+    int n = (int)(t / OH);
+    float v[V];
+    Vec<V>::get(x + (((size_t)n * H + oh / s) * W + ow / s) * C + (size_t)g * V, v);
+    Vec<V>::put(y + i * V, v);
+  }
+}
+
+template <int V>
+__global__ void __launch_bounds__(kT)
+upsample_nearest_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, int N, int H, int W, int C, int s) {
+  pdl_sync();
+  const int G = C / V, OH = H * s, OW = W * s;
+  size_t total = (size_t)N * H * W * G;
+  size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    int g = (int)(i % G);
+    size_t t = i / G;
+    int w = (int)(t % W);
+    t /= W;
+    int h = (int)(t % H);
+    int n = (int)(t / H);
+    float acc[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) acc[v] = 0.f;
+    for (int a = 0; a < s; ++a)
+      for (int b = 0; b < s; ++b) {
+        float d[V];
+        Vec<V>::get(dy + (((size_t)n * OH + h * s + a) * OW + w * s + b) * C + (size_t)g * V, d);
+#pragma unroll
+        for (int v = 0; v < V; ++v) acc[v] += d[v];
+      }
+    Vec<V>::put(dx + i * V, acc);
+  }
+}
+
+// Bilinear, align_corners=False (PyTorch's rule for an integer scale): output index o reads input indices i0 and i1
+// (i1 == i0 on the last row / column) with weights l0 and l1. Forward and backward use this one function, so the
+// backward finds exactly the taps the forward pass used.
+struct UpLerp {
+  int i0, i1;
+  float l0, l1;
+};
+__device__ __forceinline__ UpLerp up_lerp(int o, int s, int n) {
+  const float src = fmaxf(0.f, ((float)o + 0.5f) / (float)s - 0.5f);
+  UpLerp r;
+  r.i0 = (int)src;
+  r.i1 = r.i0 + (r.i0 < n - 1 ? 1 : 0);
+  r.l1 = src - (float)r.i0;
+  r.l0 = 1.f - r.l1;
+  return r;
+}
+
+template <int V>
+__global__ void __launch_bounds__(kT)
+upsample_bilinear_fwd_kernel(const float* __restrict__ x, float* __restrict__ y, int N, int H, int W, int C, int s) {
+  pdl_sync();
+  const int G = C / V, OH = H * s, OW = W * s;
+  size_t total = (size_t)N * OH * OW * G;
+  size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    int g = (int)(i % G);
+    size_t t = i / G;
+    int ow = (int)(t % OW);
+    t /= OW;
+    int oh = (int)(t % OH);
+    int n = (int)(t / OH);
+    const UpLerp r = up_lerp(oh, s, H), c = up_lerp(ow, s, W);
+    const float* base = x + (size_t)n * H * W * C + (size_t)g * V;
+    float x00[V], x01[V], x10[V], x11[V], o[V];
+    Vec<V>::get(base + ((size_t)r.i0 * W + c.i0) * C, x00);
+    Vec<V>::get(base + ((size_t)r.i0 * W + c.i1) * C, x01);
+    Vec<V>::get(base + ((size_t)r.i1 * W + c.i0) * C, x10);
+    Vec<V>::get(base + ((size_t)r.i1 * W + c.i1) * C, x11);
+#pragma unroll
+    for (int v = 0; v < V; ++v)
+      o[v] = r.l0 * (c.l0 * x00[v] + c.l1 * x01[v]) + r.l1 * (c.l0 * x10[v] + c.l1 * x11[v]);
+    Vec<V>::put(y + i * V, o);
+  }
+}
+
+template <int V>
+__global__ void __launch_bounds__(kT)
+upsample_bilinear_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, int N, int H, int W, int C, int s) {
+  pdl_sync();
+  const int G = C / V, OH = H * s, OW = W * s;
+  size_t total = (size_t)N * H * W * G;
+  size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    int g = (int)(i % G);
+    size_t t = i / G;
+    int w = (int)(t % W);
+    t /= W;
+    int h = (int)(t % H);
+    int n = (int)(t / H);
+    float acc[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) acc[v] = 0.f;
+    // an output index o has i0 = floor(max(0, (o + 0.5) / s - 0.5)): it reads input h (as i0 or i1) only when
+    // i0 is h - 1 or h, which needs s * (h - 1) <= o < s * (h + 2)
+    const int oh0 = max(0, s * (h - 1)), oh1 = min(OH, s * (h + 2));
+    const int ow0 = max(0, s * (w - 1)), ow1 = min(OW, s * (w + 2));
+    for (int oh = oh0; oh < oh1; ++oh) {
+      const UpLerp r = up_lerp(oh, s, H);
+      if (r.i0 != h && r.i1 != h) continue;
+      const float wr = (r.i0 == h ? r.l0 : 0.f) + (r.i1 == h ? r.l1 : 0.f);
+      for (int ow = ow0; ow < ow1; ++ow) {
+        const UpLerp c = up_lerp(ow, s, W);
+        if (c.i0 != w && c.i1 != w) continue;
+        const float wt = wr * ((c.i0 == w ? c.l0 : 0.f) + (c.i1 == w ? c.l1 : 0.f));
+        float d[V];
+        Vec<V>::get(dy + (((size_t)n * OH + oh) * OW + ow) * C + (size_t)g * V, d);
+#pragma unroll
+        for (int v = 0; v < V; ++v) acc[v] += wt * d[v];
+      }
+    }
+    Vec<V>::put(dx + i * V, acc);
+  }
+}
+
+// -------------------------------------------------------------------------------------------------
 // softmax cross-entropy with dense targets. One CTA: the batch dimension of every config is
 // <= a few thousand rows, and a single CTA keeps the sum order fixed.
 // -------------------------------------------------------------------------------------------------
@@ -1735,6 +1871,39 @@ dfb_status dfb_avgpool2d_bwd(const float* dy, float* dx, int N, int H, int W, in
   bool vec = C % 4 == 0 && all_aligned(dy, dx);
   POOL_DISPATCH(avgpool_bwd_kernel, (size_t)N * H * W * C, dy, dx, N, H, W, C, k, OH, OW);
   DFB_LAUNCH_CHECK("avgpool2d_bwd");
+  return DFB_OK;
+}
+
+static dfb_status upsample_geom(const char* name, int N, int H, int W, int C, int scale, int mode) {
+  DFB_REQUIRE(N > 0 && H > 0 && W > 0 && C > 0 && scale >= 1 && scale <= 8, DFB_ERR_INVALID,
+              "%s: bad geometry N=%d H=%d W=%d C=%d scale=%d (1 <= scale <= 8)", name, N, H, W, C, scale);
+  DFB_REQUIRE((long long)H * scale < (1ll << 31) && (long long)W * scale < (1ll << 31), DFB_ERR_INVALID, "%s: output too large",
+              name);
+  DFB_REQUIRE(mode == DFB_UPSAMPLE_NEAREST || mode == DFB_UPSAMPLE_BILINEAR, DFB_ERR_INVALID, "%s: bad mode %d", name, mode);
+  return DFB_OK;
+}
+dfb_status dfb_upsample2d_fwd(const float* x, float* y, int N, int H, int W, int C, int scale, int mode) {
+  DFB_INIT();
+  DFB_REQUIRE(x && y, DFB_ERR_INVALID, "upsample2d_fwd: null pointer");
+  dfb_status st = upsample_geom("upsample2d_fwd", N, H, W, C, scale, mode);
+  if (st != DFB_OK) return st;
+  bool vec = C % 4 == 0 && all_aligned(x, y);
+  size_t items = (size_t)N * H * scale * W * scale * C;
+  if (mode == DFB_UPSAMPLE_NEAREST) POOL_DISPATCH(upsample_nearest_fwd_kernel, items, x, y, N, H, W, C, scale);
+  else POOL_DISPATCH(upsample_bilinear_fwd_kernel, items, x, y, N, H, W, C, scale);
+  DFB_LAUNCH_CHECK("upsample2d_fwd");
+  return DFB_OK;
+}
+dfb_status dfb_upsample2d_bwd(const float* dy, float* dx, int N, int H, int W, int C, int scale, int mode) {
+  DFB_INIT();
+  DFB_REQUIRE(dy && dx, DFB_ERR_INVALID, "upsample2d_bwd: null pointer");
+  dfb_status st = upsample_geom("upsample2d_bwd", N, H, W, C, scale, mode);
+  if (st != DFB_OK) return st;
+  bool vec = C % 4 == 0 && all_aligned(dy, dx);
+  size_t items = (size_t)N * H * W * C;
+  if (mode == DFB_UPSAMPLE_NEAREST) POOL_DISPATCH(upsample_nearest_bwd_kernel, items, dy, dx, N, H, W, C, scale);
+  else POOL_DISPATCH(upsample_bilinear_bwd_kernel, items, dy, dx, N, H, W, C, scale);
+  DFB_LAUNCH_CHECK("upsample2d_bwd");
   return DFB_OK;
 }
 

@@ -160,6 +160,8 @@ PYBIND11_MODULE(CUDA_BACKEND, m) {
   m.attr("WLAYOUT_KRSC") = (int)DFB_WLAYOUT_KRSC;
   m.attr("DGRAD_REFERENCE") = (int)DFB_DGRAD_REFERENCE;
   m.attr("DGRAD_EXACT") = (int)DFB_DGRAD_EXACT;
+  m.attr("UPSAMPLE_NEAREST") = (int)DFB_UPSAMPLE_NEAREST;
+  m.attr("UPSAMPLE_BILINEAR") = (int)DFB_UPSAMPLE_BILINEAR;
 
   bind_vector<int32_t>(m, "Int32Vector", "Vector of int32 (shape / stride arguments)");
   bind_vector<size_t>(m, "SizeTVector", "Vector of size_t (numpy shape / stride arguments)");
@@ -515,6 +517,12 @@ PYBIND11_MODULE(CUDA_BACKEND, m) {
   });
   m.def("avgpool2d_bwd", [](const py::object& dy, const py::object& dx, int N, int H, int W, int C, int k) {
     check(dfb_avgpool2d_bwd(dptr(dy), dptr(dx), N, H, W, C, k));
+  });
+  m.def("upsample2d_fwd", [](const py::object& x, const py::object& y, int N, int H, int W, int C, int scale, int mode) {
+    check(dfb_upsample2d_fwd(dptr(x), dptr(y), N, H, W, C, scale, mode));
+  });
+  m.def("upsample2d_bwd", [](const py::object& dy, const py::object& dx, int N, int H, int W, int C, int scale, int mode) {
+    check(dfb_upsample2d_bwd(dptr(dy), dptr(dx), N, H, W, C, scale, mode));
   });
   m.def("linear_small_fwd", [](const py::object& x, const py::object& w, const py::object& bias, const py::object& y, int M, int K, int N) {
     check(dfb_linear_small_fwd(dptr(x), dptr(w), dptr(bias), dptr(y), M, K, N));

@@ -266,6 +266,8 @@ DFB_API dfb_status dfb_conv2d_workspace_floats(int N, int C, int H, int W, int K
 DFB_API dfb_status dfb_conv2d_fprop(const float* x, int x_layout, const float* w, int w_layout,
                                     float* y, int N, int C, int H, int W, int K, int R, int pad,
                                     int stride, int mode, float* workspace, size_t workspace_floats);
+/* dfb_conv2d_dgrad with DFB_DGRAD_EXACT is also the forward pass of the transposed convolution (ConvTranspose2d) whose
+ * weight is w: its input is dy [N,OH,OW,K], its output dx [N,H,W,C], its (in, out, k, k) weight is w's (K, C, R, R). */
 DFB_API dfb_status dfb_conv2d_dgrad(const float* dy, const float* w, int w_layout, float* dx, int N,
                                     int C, int H, int W, int K, int R, int pad, int stride, int mode,
                                     int dgrad_mode, float* workspace, size_t workspace_floats);
@@ -406,6 +408,16 @@ DFB_API dfb_status dfb_maxpool2d_bwd_idx(const int32_t* idx, const float* dy, fl
 /* average pooling, same geometry (the reference's avg_pool2d raises, SURVEY Q4) */
 DFB_API dfb_status dfb_avgpool2d_fwd(const float* x, float* y, int N, int H, int W, int C, int k);
 DFB_API dfb_status dfb_avgpool2d_bwd(const float* dy, float* dx, int N, int H, int W, int C, int k);
+
+/* 2-D upsampling by an integer factor 1 <= scale <= 8 on channels-last data (F.interpolate / nn.Upsample):
+ * x [N,H,W,C] -> y [N,H*scale,W*scale,C]; the backward maps dy of y's shape to dx of x's shape.
+ *   DFB_UPSAMPLE_NEAREST  : y[oh,ow] = x[oh/scale, ow/scale] (a copy, bit-exact); dx sums its scale x scale block.
+ *   DFB_UPSAMPLE_BILINEAR : align_corners=False, PyTorch's source rule src = max(0, (o + 0.5)/scale - 0.5), the last
+ *                           row / column clamped. The backward gathers: every dx element sums, in a fixed order, the
+ *                           output gradients that read it (no atomics; results do not depend on scheduling). */
+enum { DFB_UPSAMPLE_NEAREST = 0, DFB_UPSAMPLE_BILINEAR = 1 };
+DFB_API dfb_status dfb_upsample2d_fwd(const float* x, float* y, int N, int H, int W, int C, int scale, int mode);
+DFB_API dfb_status dfb_upsample2d_bwd(const float* dy, float* dx, int N, int H, int W, int C, int scale, int mode);
 
 /* Linear layers with at most 16 outputs (the classifier) in one launch each way (F.linear, functional.py:8-12; W is
  * (in, out) = K x N row-major like the reference's Linear.weight, x is M x K, bias N floats or NULL):

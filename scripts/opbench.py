@@ -18,6 +18,49 @@ import deepflows_b200  # noqa: E402,F401
 import bench  # noqa: E402
 
 
+def event_timer(m, iters, flush=None, graph=False):
+    """time_it(fn) -> microseconds per call of fn on the library's compute stream, CUDA events around each of `iters`
+    calls after 3 warm-up calls, the L2 overwritten before each (`flush`: a device Array larger than the L2, or None).
+    graph=True: 20 back-to-back calls replayed from one CUDA graph instead (no host launch cost, warm L2)."""
+    def time_it(fn):
+        for _ in range(3):
+            fn()
+        if graph:
+            reps = 20
+            m.graph_begin_capture()
+            for _ in range(reps):
+                fn()
+            g = m.graph_end_capture()
+            for _ in range(2):
+                m.graph_launch(g)
+            e0, e1 = m.event_create(), m.event_create()
+            m.event_record(e0)
+            for _ in range(5):
+                m.graph_launch(g)
+            m.event_record(e1)
+            m.event_synchronize(e1)
+            us = m.event_elapsed_ms(e0, e1) / (5 * reps) * 1e3
+            m.event_destroy(e0)
+            m.event_destroy(e1)
+            m.graph_destroy(g)
+            return us
+        tot = 0.0
+        e0, e1 = m.event_create(), m.event_create()
+        for _ in range(iters):
+            if flush is not None:
+                m.fill(flush, 0.0)
+            m.event_record(e0)
+            fn()
+            m.event_record(e1)
+            m.event_synchronize(e1)
+            tot += m.event_elapsed_ms(e0, e1)
+        m.event_destroy(e0)
+        m.event_destroy(e1)
+        return tot / iters * 1e3  # us
+
+    return time_it
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", type=int, default=256)
@@ -40,41 +83,7 @@ def main():
     flush = m.Array(64 << 20)  # 256 MB > 126 MB L2
     rng = np.random.RandomState(0)
 
-    def time_it(fn):
-        for _ in range(3):
-            fn()
-        if args.graph:
-            reps = 20
-            m.graph_begin_capture()
-            for _ in range(reps):
-                fn()
-            g = m.graph_end_capture()
-            for _ in range(2):
-                m.graph_launch(g)
-            e0, e1 = m.event_create(), m.event_create()
-            m.event_record(e0)
-            for _ in range(5):
-                m.graph_launch(g)
-            m.event_record(e1)
-            m.event_synchronize(e1)
-            us = m.event_elapsed_ms(e0, e1) / (5 * reps) * 1e3
-            m.event_destroy(e0)
-            m.event_destroy(e1)
-            m.graph_destroy(g)
-            return us
-        tot = 0.0
-        e0, e1 = m.event_create(), m.event_create()
-        for _ in range(args.iters):
-            if not args.no_flush:
-                m.fill(flush, 0.0)
-            m.event_record(e0)
-            fn()
-            m.event_record(e1)
-            m.event_synchronize(e1)
-            tot += m.event_elapsed_ms(e0, e1)
-        m.event_destroy(e0)
-        m.event_destroy(e1)
-        return tot / args.iters * 1e3  # us
+    time_it = event_timer(m, args.iters, None if args.no_flush else flush, args.graph)
 
     def dev_rand(n):
         a = m.Array(n)

@@ -9,6 +9,7 @@ deepflows_b200's host package (tests, bench.py).
   resnet_cifar    test/ResNet_CIFAR10_cuda.py:20-100  stem Conv3x3-BN-ReLU-MaxPool, 4 stages of basic
                   blocks (conv-bn-conv-bn + optional 1x1/s2 conv-bn shortcut, no ReLU inside the block),
                   mean(2), mean(2), FC
+  dcgan_generator (new, no reference script)  Linear, 3 x (ConvTranspose2d-BN-ReLU), Upsample(x2, bilinear), Conv
 """
 import types
 
@@ -297,3 +298,33 @@ def resnet_imagenet(df, device, layers=(3, 4, 6, 3), widths=(64, 128, 256, 512),
             return self.fc(x)
 
     return ResNet()
+
+
+def dcgan_generator(df, device, nz=64, widths=(256, 128, 64, 32), channels=3):
+    """A small DCGAN-style generator (a decoder: every layer makes the image larger): z (N, nz) -> Linear -> reshape to
+    (N, widths[0], 4, 4) -> 3 x [ConvTranspose2d(k4, s2, p1) -> BatchNorm2d -> ReLU] (4 -> 8 -> 16 -> 32 px) ->
+    Upsample(x2, bilinear) -> Conv2d(k3, p1) to `channels` -> (N, channels, 64, 64)."""
+    nn = df.nn
+
+    class Generator(nn.Module):
+        def __init__(self):
+            super().__init__()
+            self.fc = nn.Linear(nz, widths[0] * 16, device=device)
+            self.ups = []
+            for i, (cin, cout) in enumerate(zip(widths[:-1], widths[1:])):
+                up = (nn.ConvTranspose2d(cin, cout, kernel_size=4, padding=1, stride=2, bias=False, device=device),
+                      nn.BatchNorm2d(cout, device=device))
+                setattr(self, "up%d" % (i + 1), up[0])
+                setattr(self, "bn%d" % (i + 1), up[1])
+                self.ups.append(up)
+            self.relu = nn.ReLU()
+            self.upsample = nn.Upsample(scale_factor=2, mode="bilinear")
+            self.out = nn.Conv2d(widths[-1], channels, kernel_size=3, padding=1, device=device)
+
+        def forward(self, z):
+            x = self.fc(z).reshape(z.shape[0], widths[0], 4, 4)
+            for conv, bn in self.ups:
+                x = self.relu(bn(conv(x)))
+            return self.out(self.upsample(x))
+
+    return Generator()
