@@ -12,8 +12,9 @@ What is different: gradients that were broadcast in the forward pass are reduced
 (the reference round-trips them through numpy, [462-483]); gradient buffers are created when the first
 gradient arrives instead of a zero-fill per node [134]; `FusedOperator` lets one node (conv2d,
 batch-norm, pooling, cross-entropy in nn/functional.py) return the gradients of all its inputs from a
-single fused backward kernel.
+single fused backward kernel; `cat` (absent in the reference) is such a node.
 """
+import builtins
 from typing import Any, List, Optional, Tuple, Type, Union  # noqa: F401  (re-exported: the scripts star-import this module)
 
 import numpy  # noqa: F401
@@ -25,7 +26,7 @@ from .backend_selection import Device, backend_api, BackendTensor, default_devic
 __all__ = [
     "Graph", "Tensor", "UnaryOperator", "BinaryOperator", "FusedOperator", "add", "sub", "mul", "div", "pow",
     "matmul", "sum", "mean", "max", "exp", "log", "maximum", "sqrt", "square", "Reshape", "transpose",
-    "get_slice", "empty", "zeros", "ones", "randn", "rand", "uniform",
+    "get_slice", "cat", "empty", "zeros", "ones", "randn", "rand", "uniform",
     # what `from DeepFlows.tensor import *` also brings into a script with the reference (it defines no __all__)
     "np", "numpy", "is_grad_enable", "no_grad", "Device", "backend_api", "BackendTensor", "default_device",
     "Any", "List", "Optional", "Tuple", "Type", "Union",
@@ -714,6 +715,87 @@ class get_slice(UnaryOperator):
         full = backend_api.zeros(x.shape, device=x.device)
         full[self.key] = grad
         return full
+
+
+_CONCAT_MAX_SOURCES = 8   # include/dfb200.h: DFB_CONCAT_MAX_SOURCES
+
+
+def _nhwc(handle, n, c, h, w, device):
+    return BackendTensor.make((n, c, h, w), (h * w * c, 1, w * c, c), device, handle)
+
+
+class _cat(FusedOperator):
+    """Concatenation along `dim` as one graph node. 4-d inputs along dim 1 (at most 8 of them, on a device with
+    concat_channels_fwd) take one channels-last kernel each way: the output is channels-last, and so is every input
+    gradient - the layout a convolution's dgrad epilogue needs to add the gradient its input already holds. Everything else
+    writes a compact output with one strided setitem per input and slices the gradient back out."""
+
+    def __init__(self, tensors, dim):
+        self.dim = dim
+        x = tensors[0]
+        self._fused = (x.ndim == 4 and dim == 1 and len(tensors) <= _CONCAT_MAX_SOURCES
+                       and x.device.has("concat_channels_fwd"))
+        super().__init__(*tensors)
+
+    def forward(self, *inputs):
+        datas = [t.data for t in inputs]
+        dev = datas[0].device
+        self._sizes = [d.shape[self.dim] for d in datas]
+        self._ndim = datas[0].ndim
+        shape = list(datas[0].shape)
+        shape[self.dim] = builtins.sum(self._sizes)
+        if self._fused:
+            xs = [d.channels_last() for d in datas]   # a pending relu(bn(..)) is written here, once
+            n, c, h, w = shape
+            y = dev.Array(n * h * w * c)
+            dev.concat_channels_fwd([x._handle for x in xs], self._sizes, y, n * h * w)
+            return _nhwc(y, n, c, h, w, dev)
+        out = BackendTensor.make(shape, device=dev)
+        for key, d in zip(self._slices(), datas):
+            out[key] = d
+        return out
+
+    def _slices(self):
+        start = 0
+        for size in self._sizes:
+            yield tuple(slice(start, start + size) if a == self.dim else slice(None) for a in range(self._ndim))
+            start += size
+
+    def backward_all(self, grad, needs):
+        if not self._fused:
+            return [grad[key].compact() if need else None for key, need in zip(self._slices(), needs)]
+        n, _, h, w = grad.shape
+        dev = grad.device
+        gy = grad.channels_last()
+        outs = [dev.Array(n * h * w * c) if need else None for c, need in zip(self._sizes, needs)]
+        dev.concat_channels_bwd(gy._handle, outs, self._sizes, n * h * w)
+        return [_nhwc(o, n, c, h, w, dev) if o is not None else None for o, c in zip(outs, self._sizes)]
+
+
+def cat(tensors, dim=0):
+    """Concatenation of a non-empty sequence of tensors along `dim`, torch.cat's contract: the tensors live on one device,
+    have the same number of axes and the same size on every axis but `dim` (negative `dim` counts from the end).
+    ValueError for an empty sequence or mismatched tensors, IndexError for `dim` out of range. One graph node: a tensor
+    listed twice receives the sum of both slices' gradients."""
+    tensors = list(tensors)
+    if not tensors:
+        raise ValueError("cat: expected a non-empty sequence of tensors")
+    if not all(isinstance(t, Tensor) for t in tensors):
+        raise TypeError("cat: expected a sequence of Tensors")
+    first = tensors[0]
+    nd = first.ndim
+    if not -nd <= dim < nd:
+        raise IndexError("cat: dim %d is out of range for %d-d tensors" % (dim, nd))
+    dim %= nd
+    for i, t in enumerate(tensors):
+        if t.ndim != nd:
+            raise ValueError("cat: tensor %d has %d dimensions, tensor 0 has %d" % (i, t.ndim, nd))
+        if t.device != first.device:
+            raise ValueError("cat: tensor %d is on %s, tensor 0 on %s" % (i, t.device, first.device))
+        if any(a != b for ax, (a, b) in enumerate(zip(t.shape, first.shape)) if ax != dim):
+            raise ValueError("cat: tensor %d has shape %s, tensor 0 has %s: sizes must match except along dim %d"
+                             % (i, t.shape, first.shape, dim))
+    return _cat(tensors, dim)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -1167,6 +1167,48 @@ upsample_bilinear_bwd_kernel(const float* __restrict__ dy, float* __restrict__ d
 }
 
 // -------------------------------------------------------------------------------------------------
+// channel concatenation on NHWC: slice s is a [rows, width[s]] matrix and occupies columns off[s] .. off[s] + width[s]
+// of y [rows, C]. The slice table is a kernel parameter, so a captured graph keeps it in the kernel node (no device
+// table, no upload). blockIdx.y picks the slice; its CTAs walk it with a grid-stride loop, kConcatUnroll vectors per
+// thread loaded before any is stored: the slice side is read / written contiguously, the y side in row segments.
+// -------------------------------------------------------------------------------------------------
+constexpr int kConcatUnroll = 4;
+struct ConcatSlices {
+  float* p[DFB_CONCAT_MAX_SOURCES];   // the source (forward) or its gradient (backward)
+  int off[DFB_CONCAT_MAX_SOURCES];
+  int width[DFB_CONCAT_MAX_SOURCES];
+};
+
+template <int V, bool BWD>
+__global__ void __launch_bounds__(kT)
+concat_channels_kernel(const __grid_constant__ ConcatSlices t, float* __restrict__ y, int C, long long rows) {
+  pdl_sync();
+  const int s = blockIdx.y;
+  float* __restrict__ part = t.p[s];
+  float* __restrict__ ys = y + t.off[s];
+  const int G = t.width[s] / V;
+  const size_t total = (size_t)rows * G;
+  const size_t stride = (size_t)gridDim.x * blockDim.x * kConcatUnroll;
+  for (size_t base = (size_t)blockIdx.x * blockDim.x * kConcatUnroll + threadIdx.x; base < total; base += stride) {
+    float v[kConcatUnroll][V];
+#pragma unroll
+    for (int u = 0; u < kConcatUnroll; ++u) {
+      const size_t i = base + (size_t)u * blockDim.x;
+      if (i >= total) break;
+      const size_t r = i / G;
+      Vec<V>::get(BWD ? ys + r * C + (i - r * G) * V : part + i * V, v[u]);
+    }
+#pragma unroll
+    for (int u = 0; u < kConcatUnroll; ++u) {
+      const size_t i = base + (size_t)u * blockDim.x;
+      if (i >= total) break;
+      const size_t r = i / G;
+      Vec<V>::put(BWD ? part + i * V : ys + r * C + (i - r * G) * V, v[u]);
+    }
+  }
+}
+
+// -------------------------------------------------------------------------------------------------
 // softmax cross-entropy with dense targets. One CTA: the batch dimension of every config is
 // <= a few thousand rows, and a single CTA keeps the sum order fixed.
 // -------------------------------------------------------------------------------------------------
@@ -1905,6 +1947,57 @@ dfb_status dfb_upsample2d_bwd(const float* dy, float* dx, int N, int H, int W, i
   else POOL_DISPATCH(upsample_bilinear_bwd_kernel, items, dy, dx, N, H, W, C, scale);
   DFB_LAUNCH_CHECK("upsample2d_bwd");
   return DFB_OK;
+}
+
+// One launch for the slices whose pointer is not null (the backward skips inputs that need no gradient); y is the
+// concatenated matrix, read by the backward and written by the forward.
+static dfb_status concat_channels(const char* name, float* const* parts, const int* widths, int count, float* y,
+                                  long long rows, bool bwd) {
+  DFB_REQUIRE(count >= 1 && count <= DFB_CONCAT_MAX_SOURCES, DFB_ERR_INVALID, "%s: %d sources (1 to %d)", name, count,
+              DFB_CONCAT_MAX_SOURCES);
+  DFB_REQUIRE(parts && widths && y, DFB_ERR_INVALID, "%s: null pointer", name);
+  DFB_REQUIRE(rows > 0, DFB_ERR_INVALID, "%s: rows must be positive, got %lld", name, rows);
+  ConcatSlices t = {};
+  int n = 0, widest = 0;
+  long long C = 0;
+  bool vec = all_aligned(y);
+  for (int i = 0; i < count; ++i) {
+    DFB_REQUIRE(widths[i] > 0, DFB_ERR_INVALID, "%s: width %d of source %d must be positive", name, widths[i], i);
+    vec = vec && widths[i] % 4 == 0 && all_aligned(parts[i]);
+    if (parts[i]) {
+      t.p[n] = parts[i];
+      t.off[n] = (int)C;
+      t.width[n] = widths[i];
+      widest = std::max(widest, widths[i]);
+      ++n;
+    }
+    C += widths[i];
+    DFB_REQUIRE(C < (1ll << 31), DFB_ERR_INVALID, "%s: %lld channels or more (limit 2^31 - 1)", name, C);
+  }
+  if (n == 0) return DFB_OK;
+  const int V = vec ? 4 : 1;
+  const unsigned per_slice = std::max(1u, (unsigned)(sm_count() * 8 / n));
+  const size_t vectors = ((size_t)rows * (widest / V) + kConcatUnroll - 1) / kConcatUnroll;
+  const dim3 grid(std::min(bw_grid(vectors, kT), per_slice), n);
+  if (bwd) {
+    if (vec) launch_k(concat_channels_kernel<4, true>, grid, kT, 0, compute_stream(), t, y, (int)C, rows);
+    else launch_k(concat_channels_kernel<1, true>, grid, kT, 0, compute_stream(), t, y, (int)C, rows);
+  } else {
+    if (vec) launch_k(concat_channels_kernel<4, false>, grid, kT, 0, compute_stream(), t, y, (int)C, rows);
+    else launch_k(concat_channels_kernel<1, false>, grid, kT, 0, compute_stream(), t, y, (int)C, rows);
+  }
+  DFB_LAUNCH_CHECK(name);
+  return DFB_OK;
+}
+dfb_status dfb_concat_channels_fwd(const float* const* srcs, const int* widths, int count, float* y, long long rows) {
+  DFB_INIT();
+  for (int i = 0; srcs && i < count && i < DFB_CONCAT_MAX_SOURCES; ++i)
+    DFB_REQUIRE(srcs[i], DFB_ERR_INVALID, "concat_channels_fwd: source %d is null", i);
+  return concat_channels("concat_channels_fwd", const_cast<float* const*>(srcs), widths, count, y, rows, false);
+}
+dfb_status dfb_concat_channels_bwd(const float* dy, float* const* dsrcs, const int* widths, int count, long long rows) {
+  DFB_INIT();
+  return concat_channels("concat_channels_bwd", dsrcs, widths, count, const_cast<float*>(dy), rows, true);
 }
 
 dfb_status dfb_linear_small_fwd(const float* x, const float* w, const float* bias, float* y, int M, int K, int N) {

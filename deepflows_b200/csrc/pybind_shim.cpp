@@ -586,6 +586,21 @@ PYBIND11_MODULE(CUDA_BACKEND, m) {
     if (s.size() != sizes.size() || d.size() != sizes.size()) throw py::value_error("multi_copy: table lengths differ");
     check(dfb_multi_copy((const float* const*)s.data(), d.data(), sizes.data(), (int)sizes.size()));
   });
+  // the library checks the tables (count, null sources, widths)
+  m.def("concat_channels_fwd", [ptr_table](const py::sequence& srcs, const std::vector<int>& widths, const py::object& y,
+                                           long long rows) {
+    std::vector<float*> s;
+    ptr_table(srcs, &s, true);
+    if (s.size() != widths.size()) throw py::value_error("concat_channels_fwd: table lengths differ");
+    check(dfb_concat_channels_fwd((const float* const*)s.data(), widths.data(), (int)s.size(), dptr(y), rows));
+  });
+  m.def("concat_channels_bwd", [ptr_table](const py::object& dy, const py::sequence& dsrcs, const std::vector<int>& widths,
+                                           long long rows) {
+    std::vector<float*> d;
+    ptr_table(dsrcs, &d, true);
+    if (d.size() != widths.size()) throw py::value_error("concat_channels_bwd: table lengths differ");
+    check(dfb_concat_channels_bwd(dptr(dy), d.data(), widths.data(), (int)d.size(), rows));
+  });
 
   // ---- pinned host buffers + async copies (input pipeline / bench e2e) ------------------------------
   m.def("pinned_empty", [](size_t n) {

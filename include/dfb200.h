@@ -419,6 +419,18 @@ enum { DFB_UPSAMPLE_NEAREST = 0, DFB_UPSAMPLE_BILINEAR = 1 };
 DFB_API dfb_status dfb_upsample2d_fwd(const float* x, float* y, int N, int H, int W, int C, int scale, int mode);
 DFB_API dfb_status dfb_upsample2d_bwd(const float* dy, float* dx, int N, int H, int W, int C, int scale, int mode);
 
+/* Channel concatenation of channels-last tensors (torch.cat(dim=1) on NHWC, the U-Net skip connection): source i is a
+ * [rows, widths[i]] matrix (rows = N*H*W) and occupies columns off_i .. off_i + widths[i] of y [rows, C], where
+ * off_i = widths[0] + ... + widths[i-1] and C = the sum of the widths (< 2^31). 1 <= count <= DFB_CONCAT_MAX_SOURCES:
+ * the pointer table travels as a kernel parameter, so a captured graph gets no copy node for it.
+ *   fwd: y[:, off_i : off_i + widths[i]] = srcs[i]
+ *   bwd: dsrcs[i] = dy[:, off_i : off_i + widths[i]]; a null dsrcs[i] (an input that needs no gradient) is skipped.
+ * One launch each way; the kernels copy, so results are bit-exact. The pointer tables are HOST arrays. */
+#define DFB_CONCAT_MAX_SOURCES 8
+DFB_API dfb_status dfb_concat_channels_fwd(const float* const* srcs, const int* widths, int count, float* y, long long rows);
+DFB_API dfb_status dfb_concat_channels_bwd(const float* dy, float* const* dsrcs, const int* widths, int count,
+                                           long long rows);
+
 /* Linear layers with at most 16 outputs (the classifier) in one launch each way (F.linear, functional.py:8-12; W is
  * (in, out) = K x N row-major like the reference's Linear.weight, x is M x K, bias N floats or NULL):
  *   fwd: y = x . W + bias          bwd: dx = dy . W^T, dw = x^T . dy, db = column sums of dy (each may be NULL) */

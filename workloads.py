@@ -10,6 +10,8 @@ deepflows_b200's host package (tests, bench.py).
                   blocks (conv-bn-conv-bn + optional 1x1/s2 conv-bn shortcut, no ReLU inside the block),
                   mean(2), mean(2), FC
   dcgan_generator (new, no reference script)  Linear, 3 x (ConvTranspose2d-BN-ReLU), Upsample(x2, bilinear), Conv
+  unet            (new, no reference script)  encoder levels of 2 x (Conv-BN-ReLU) with MaxPool between them, decoder
+                  levels of ConvTranspose2d(k2, s2), cat with the skip, 2 x (Conv-BN-ReLU); 1x1 Conv head
 """
 import types
 
@@ -328,3 +330,56 @@ def dcgan_generator(df, device, nz=64, widths=(256, 128, 64, 32), channels=3):
             return self.out(self.upsample(x))
 
     return Generator()
+
+
+def unet(df, device, in_channels=3, out_channels=3, widths=(32, 64, 128, 256)):
+    """A U-Net (encoder-decoder with skip connections): len(widths) levels. Each encoder level is
+    [Conv3x3(p1, bias-free) -> BatchNorm2d -> ReLU] x 2, with MaxPool2d(2) between levels. Each decoder level is
+    ConvTranspose2d(k2, s2, bias-free) from widths[i+1] to widths[i], `cat([up, skip], dim=1)` with the encoder output of the
+    same level, then [Conv3x3 -> BN -> ReLU] x 2 from 2 * widths[i] to widths[i]. A 1x1 Conv2d maps to `out_channels`.
+    H and W must be divisible by 2 ** (len(widths) - 1); the output has the input's size."""
+    nn, tensor = df.nn, df.tensor
+
+    class DoubleConv(nn.Module):
+        def __init__(self, cin, cout):
+            super().__init__()
+            self.conv1 = nn.Conv2d(cin, cout, kernel_size=3, padding=1, bias=False, device=device)
+            self.bn1 = nn.BatchNorm2d(cout, device=device)
+            self.conv2 = nn.Conv2d(cout, cout, kernel_size=3, padding=1, bias=False, device=device)
+            self.bn2 = nn.BatchNorm2d(cout, device=device)
+            self.relu = nn.ReLU()
+
+        def forward(self, x):
+            return self.relu(self.bn2(self.conv2(self.relu(self.bn1(self.conv1(x))))))
+
+    class UNet(nn.Module):
+        def __init__(self):
+            super().__init__()
+            self.down = []
+            for i, (cin, cout) in enumerate(zip((in_channels,) + tuple(widths[:-1]), widths)):
+                self.down.append(DoubleConv(cin, cout))
+                setattr(self, "down%d" % i, self.down[-1])
+            self.pool = nn.MaxPool2d(kernel_size=2, stride=2)
+            self.up = []
+            for i in reversed(range(len(widths) - 1)):
+                up = (nn.ConvTranspose2d(widths[i + 1], widths[i], kernel_size=2, stride=2, bias=False, device=device),
+                      DoubleConv(2 * widths[i], widths[i]))
+                setattr(self, "up%d" % i, up[0])
+                setattr(self, "dec%d" % i, up[1])
+                self.up.append(up)
+            self.head = nn.Conv2d(widths[0], out_channels, kernel_size=1, device=device)
+
+        def forward(self, x):
+            levels = len(widths)
+            if x.shape[2] % 2 ** (levels - 1) or x.shape[3] % 2 ** (levels - 1):
+                raise ValueError("unet: H and W (%d, %d) must be divisible by %d" % (x.shape[2], x.shape[3], 2 ** (levels - 1)))
+            skips = []
+            for i, block in enumerate(self.down):
+                x = block(x if i == 0 else self.pool(x))
+                skips.append(x)
+            x = skips.pop()
+            for upconv, block in self.up:
+                x = block(tensor.cat([upconv(x), skips.pop()], dim=1))
+            return self.head(x)
+
+    return UNet()
